@@ -2,6 +2,7 @@
 """bench.py — adversarial images / second, MI-FGSM ResNet-50 224^2 10 iterations (BASELINE.json `metric`).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            our arm (N>1: launched by torch.distributed.run)
+    python bench.py [...] --dump-outputs DIR                       … and the last timed step's perturbation → DIR/delta.npy
     python bench.py --impl reference [...]                          the reference's CPU path (oracle port) on the host cores
     python bench.py --kernels                                       per-kernel roofline table  (gpurun_out/kernels.json)
     python bench.py --sweep                                         fused-update tuning sweep  (gpurun_out/sweep.json)
@@ -47,7 +48,14 @@ def parse():
     p.add_argument("--no-cpu-baseline", action="store_true")
     p.add_argument("--cpu-worker", default="", help="internal: 'sample_b,steps,warmup' → JSON on stdout")
     p.add_argument("--no-eager-gpu", action="store_true")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default="",
+                   help="after the timed steps, write the perturbation the last timed step returned to DIR/delta.npy (float32)")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.kernels or args.sweep):
+        p.error("--dump-outputs applies to the attack timed by `--impl ours` (not --kernels / --sweep)")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -388,6 +396,8 @@ def run_ours(args, rank, local_rank, world, dist):
         sts = list(atk._graphs.values())
         launches += sts[-1].get("kernels_per_replay", 0) * args.epoch * args.steps
     last_timed = keep.get("d")
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_timed, rank, world, dist)
 
     # -- roofline of the tail -----------------------------------------------------------------------------------------
     k_ms, ms_ev = tail_events(atk, x_dev, y_dev, max(2, args.steps // 2), dist, device)
@@ -510,6 +520,29 @@ def run_ours(args, rank, local_rank, world, dist):
         }
         line.update(extra)
         print(json.dumps(line), flush=True)
+
+
+DUMP_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(out_dir, delta, rank, world, dist):
+    """--dump-outputs: the perturbation the last timed step returned (every rank's shard, in rank order) as DIR/delta.npy in
+    float32. The inputs are seeded, so two builds run with the same arguments can be compared element for element. An output
+    larger than DUMP_BYTES is written as a fixed sample of its flattened elements (distinct indices drawn with seed 0, in
+    increasing order), and those indices go to DIR/delta_index.npy (float64, exact below 2^53)."""
+    if dist is not None:
+        parts = [torch.empty_like(delta) for _ in range(world)]
+        dist.all_gather(parts, delta.contiguous())
+        delta = torch.cat(parts)
+    if rank != 0:
+        return
+    d = delta.float().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    if d.nbytes > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(d.size, DUMP_BYTES // 16, replace=False))   # 4 + 8 bytes per sample
+        d = d.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, "delta_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "delta.npy"), d)
 
 
 def workload_config(args, world, atk=None, x_dev=None):

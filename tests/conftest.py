@@ -9,11 +9,13 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
+# a checkout of the unmodified Trustworthy-AI-Group/TransferAttack, for the tests marked `reference`
+REF_ROOT = os.environ.get("TRANSFERATTACK_REFERENCE", "")
 
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
+    config.addinivalue_line("markers", "reference: needs a checkout of the unmodified reference in $TRANSFERATTACK_REFERENCE")
 
 
 def pytest_collection_modifyitems(config, items):
@@ -26,8 +28,8 @@ def pytest_collection_modifyitems(config, items):
     for item in items:
         if "gpu" in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
-        if "reference" in item.keywords and not os.path.isdir("/root/reference/transferattack"):
-            item.add_marker(pytest.mark.skip(reason="/root/reference absent"))
+        if "reference" in item.keywords and not (REF_ROOT and os.path.isdir(os.path.join(REF_ROOT, "transferattack"))):
+            item.add_marker(pytest.mark.skip(reason="no reference checkout ($TRANSFERATTACK_REFERENCE)"))
 
 
 def load_golden(name):

@@ -1,8 +1,6 @@
-"""Generate tests/golden/*.npz by running the UNMODIFIED reference (imported from /root/reference) on CPU.
+"""Generate tests/golden/*.npz by running the UNMODIFIED reference (a checkout of Trustworthy-AI-Group/TransferAttack) on CPU:
 
-Run in the build container only (the reference does not exist on the GPU box):
-
-    python tests/golden/make_golden.py
+    TRANSFERATTACK_REFERENCE=<checkout> python tests/golden/make_golden.py
 
 Shims (SURVEY.md §8c; no reference source is edited or copied):
   * `timm` is absent → a stub module with `list_models()` is inserted before import;
@@ -24,10 +22,12 @@ import torch.nn as nn
 import torchvision
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = "/root/reference"
+REF = os.environ.get("TRANSFERATTACK_REFERENCE", "")
 
 
 def import_reference():
+    if not os.path.isdir(os.path.join(REF, "transferattack")):
+        sys.exit("set TRANSFERATTACK_REFERENCE to a checkout of the unmodified reference")
     if "timm" not in sys.modules:
         try:
             import timm  # noqa: F401

@@ -6,7 +6,7 @@ import numpy as np
 import torch
 import torch.nn as nn
 
-REF_ROOT = "/root/reference"
+from conftest import REF_ROOT  # noqa: F401  (a checkout of the unmodified reference, or "")
 
 
 class TinyNet(nn.Module):
@@ -48,7 +48,7 @@ def make_attack(pkg, name, net_or_list, wrap=None, ens=None, **kw):
 
 
 def import_reference():
-    """The unmodified reference package (build container only)."""
+    """The unmodified reference package (from $TRANSFERATTACK_REFERENCE)."""
     if "timm" not in sys.modules:
         try:
             import timm  # noqa: F401

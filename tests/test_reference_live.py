@@ -1,7 +1,7 @@
-"""Build-container only (needs /root/reference): the LIVE unmodified reference as the judge of
+"""Needs a checkout of the unmodified reference in $TRANSFERATTACK_REFERENCE (skipped without one): the LIVE reference as the judge of
   (1) oracle/torch_ref.py — the eager restatement must reproduce the reference's perturbation bit for bit, and
   (2) the drop-in boundary — the reference's OWN plugin files, loaded on top of this package's Attack/utils through
-      transferattack_b200.compat (kernels replaced by the oracle stand-in on this GPU-less box), must produce exactly what
+      transferattack_b200.compat (kernels replaced by the oracle stand-in, so no GPU is needed), must produce exactly what
       they produce on the reference's own base class (SURVEY.md Appendix B.2 regression matrix)."""
 import random
 
