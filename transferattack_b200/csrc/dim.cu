@@ -296,7 +296,7 @@ int ta_dim_fwd(const float* x, float* out, int planes, int S, int rnd, int R, in
   const int a_rows = gm.src_rows_max > gm.t2_rows_max ? gm.src_rows_max : gm.t2_rows_max;
   const size_t smem = align16((size_t)a_rows * S * 4) + sizeof(Tap) * (size_t)(S + rnd) +
                       sizeof(float) * ((size_t)gm.src_rows_max * rnd + (size_t)gm.y1_rows_max * rnd);
-  TA_REQUIRE(smem <= 200 * 1024, "ta_dim_fwd: image size S=%d needs %zu B of shared memory per CTA", S, smem);
+  TA_REQUIRE(smem <= 200 * 1024, "ta_dim_fwd: image size S=%d needs %zu B of shared memory per CTA, more than the 204800 B limit", S, smem);
   auto k = can_tma ? dim_fwd_kernel<true> : dim_fwd_kernel<false>;
   static SmemOptIn optin_tma = {}, optin_ldg = {};
   rc = ensure_dyn_smem("ta_dim_fwd", k, smem, can_tma ? optin_tma : optin_ldg);
@@ -318,7 +318,7 @@ int ta_dim_bwd(const float* gout, float* gin, int planes, int S, int rnd, int R,
   const size_t u_elems = (size_t)gm.y1_rows_max * S > (size_t)RB * rnd ? (size_t)gm.y1_rows_max * S : (size_t)RB * rnd;
   const size_t smem = sizeof(Tap) * (size_t)(S + rnd) + sizeof(int) * (size_t)(2 * R + 2 * S) +
                       sizeof(float) * (u_elems + (size_t)gm.y1_rows_max * rnd);
-  TA_REQUIRE(smem <= 200 * 1024, "ta_dim_bwd: image size S=%d needs %zu B of shared memory per CTA", S, smem);
+  TA_REQUIRE(smem <= 200 * 1024, "ta_dim_bwd: image size S=%d needs %zu B of shared memory per CTA, more than the 204800 B limit", S, smem);
   static SmemOptIn optin = {};
   rc = ensure_dyn_smem("ta_dim_bwd", dim_bwd_kernel, smem, optin);
   if (rc != TA_OK) return rc;
@@ -370,23 +370,33 @@ int ta_dim_pack_build(void* host_pack, int S, int rnd, int R, int pad_top, int p
   if (!identity) {
     const int rc = check_geom("ta_dim_pack_build", 1, S, rnd, R, pad_top, pad_left);
     if (rc != TA_OK) return rc;
-    if (!dim_direct_ok(S, rnd, R)) { set_error("ta_dim_pack_build: S=%d R=%d beyond the direct kernels' tables", S, R); return TA_EUNSUPPORTED; }
+    if (!dim_direct_ok(S, rnd, R)) { set_error("ta_dim_pack_build: S=%d R=%d beyond the direct kernels' tables (S <= %d, R <= %d)", S, R, kDimMaxS, kDimMaxR); return TA_EUNSUPPORTED; }
   }
   return dim_pack_build(reinterpret_cast<DimPack*>(host_pack), S, rnd, R, pad_top, pad_left, identity);
 }
 
 int ta_dim_fwd_dyn(const float* x, float* out, int planes, int S, int R, const void* packs, int n_packs, const int* it,
                    ta_stream_t stream) {
-  TA_REQUIRE(x && out && packs && it && n_packs > 0 && planes > 0 && planes <= 65535, "ta_dim_fwd_dyn: bad arguments");
-  if (!dim_direct_ok(S, S, R) || !aligned16(packs)) { set_error("ta_dim_fwd_dyn: S=%d R=%d unsupported or misaligned packs", S, R); return TA_EUNSUPPORTED; }
+  TA_REQUIRE(x && out && packs && it && n_packs > 0 && planes > 0, "ta_dim_fwd_dyn: bad arguments");
+  TA_REQUIRE(planes <= 65535, "ta_dim_fwd_dyn: planes=%d exceeds 65535", planes);
+  if (!aligned16(packs)) { set_error("ta_dim_fwd_dyn: packs are not 16-byte aligned"); return TA_EUNSUPPORTED; }
+  if (!dim_direct_ok(S, S, R)) {
+    set_error("ta_dim_fwd_dyn: S=%d R=%d beyond the direct kernels' tables (S <= %d, R <= %d)", S, R, kDimMaxS, kDimMaxR);
+    return TA_EUNSUPPORTED;
+  }
   return dim_fwd_dyn(x, out, planes, S, R, reinterpret_cast<const DimPack*>(packs), n_packs, it,
                      (S % 4 == 0) && aligned16(x) && tune_get("dim.tma", 1) != 0, (cudaStream_t)stream);
 }
 
 int ta_dim_bwd_dyn(const float* gout, float* gin, int planes, int S, int R, const void* packs, int n_packs, const int* it,
                    ta_stream_t stream) {
-  TA_REQUIRE(gout && gin && packs && it && n_packs > 0 && planes > 0 && planes <= 65535, "ta_dim_bwd_dyn: bad arguments");
-  if (!dim_direct_ok(S, S, R) || !aligned16(packs)) { set_error("ta_dim_bwd_dyn: S=%d R=%d unsupported or misaligned packs", S, R); return TA_EUNSUPPORTED; }
+  TA_REQUIRE(gout && gin && packs && it && n_packs > 0 && planes > 0, "ta_dim_bwd_dyn: bad arguments");
+  TA_REQUIRE(planes <= 65535, "ta_dim_bwd_dyn: planes=%d exceeds 65535", planes);
+  if (!aligned16(packs)) { set_error("ta_dim_bwd_dyn: packs are not 16-byte aligned"); return TA_EUNSUPPORTED; }
+  if (!dim_direct_ok(S, S, R)) {
+    set_error("ta_dim_bwd_dyn: S=%d R=%d beyond the direct kernels' tables (S <= %d, R <= %d)", S, R, kDimMaxS, kDimMaxR);
+    return TA_EUNSUPPORTED;
+  }
   return dim_bwd_dyn(gout, gin, planes, S, R, reinterpret_cast<const DimPack*>(packs), n_packs, it,
                      (S % 4 == 0) && aligned16(gout) && tune_get("dim.tma", 1) != 0, (cudaStream_t)stream);
 }

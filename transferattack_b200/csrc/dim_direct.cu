@@ -1231,7 +1231,7 @@ int dim_fwd_dyn(const float* x, float* out, int planes, int S, int R, const DimP
     count_launch();
     return check_launch("ta_dim_fwd_dyn[sep]");
   }
-  TA_REQUIRE(smem <= 200 * 1024, "ta_dim_fwd_dyn: image size S=%d needs %zu B of shared memory per CTA", S, smem);
+  TA_REQUIRE(smem <= 200 * 1024, "ta_dim_fwd_dyn: image size S=%d needs %zu B of shared memory per CTA, more than the 204800 B limit", S, smem);
   auto k = tma ? dim_fwd_direct_kernel<1, true, FwdTabDyn, true> : dim_fwd_direct_kernel<1, false, FwdTabDyn, true>;
   static SmemOptIn optin[2] = {};
   const int rc = ensure_dyn_smem("ta_dim_fwd_dyn", k, smem, optin[tma ? 0 : 1]);
@@ -1257,7 +1257,7 @@ int dim_bwd_dyn(const float* gout, float* gin, int planes, int S, int R, const D
     count_launch();
     return check_launch("ta_dim_bwd_dyn[sep]");
   }
-  TA_REQUIRE(smem <= 200 * 1024, "ta_dim_bwd_dyn: image size S=%d needs %zu B of shared memory per CTA", S, smem);
+  TA_REQUIRE(smem <= 200 * 1024, "ta_dim_bwd_dyn: image size S=%d needs %zu B of shared memory per CTA, more than the 204800 B limit", S, smem);
   auto k = tma ? dim_bwd_direct_kernel<true, true> : dim_bwd_direct_kernel<false, true>;
   static SmemOptIn optin[2] = {};
   const int rc = ensure_dyn_smem("ta_dim_bwd_dyn", k, smem, optin[tma ? 0 : 1]);
@@ -1365,7 +1365,7 @@ int dim_fwd_direct(const float* x, float* out, int planes, int S, int rnd, int R
     return check_launch("ta_dim_fwd[sep]");
   }
   const size_t smem = ((sizeof(float) * ((size_t)a_rows * S + (size_t)(c_rows + 1) * (rnd + 1)) + 15) & ~(size_t)15) + 16 * (size_t)(c_rows + RB);
-  TA_REQUIRE(smem <= 200 * 1024, "ta_dim_fwd: image size S=%d needs %zu B of shared memory per CTA", S, smem);
+  TA_REQUIRE(smem <= 200 * 1024, "ta_dim_fwd: image size S=%d needs %zu B of shared memory per CTA, more than the 204800 B limit", S, smem);
   static SmemOptIn optin[40] = {};
 #define TA_DIM_FWD_LAUNCH(MODE_, SLOT_)                                                                             \
   do {                                                                                                              \
@@ -1451,7 +1451,7 @@ int dim_bwd_direct(const float* gout, float* gin, int planes, int S, int rnd, in
     const int wext = cmax - 2 > 1 ? cmax - 2 : 1;
     const size_t smem_g = ((sizeof(float) * ((size_t)u_rows * S + (size_t)g_rows * rnd) + 15) & ~(size_t)15) +
                           16 * (size_t)(g_rows + RB) + sizeof(float) * (size_t)wext * (g_rows + RB);
-    TA_REQUIRE(smem_g <= 200 * 1024, "ta_dim_bwd: image size S=%d needs %zu B of shared memory per CTA", S, smem_g);
+    TA_REQUIRE(smem_g <= 200 * 1024, "ta_dim_bwd: image size S=%d needs %zu B of shared memory per CTA, more than the 204800 B limit", S, smem_g);
     auto kg = tma ? dim_bwd_gather_kernel<true> : dim_bwd_gather_kernel<false>;
     static SmemOptIn optin_g[2] = {};
     const int rcg = ensure_dyn_smem("ta_dim_bwd", kg, smem_g, optin_g[tma ? 0 : 1]);
@@ -1462,7 +1462,7 @@ int dim_bwd_direct(const float* gout, float* gin, int planes, int S, int rnd, in
     return check_launch("ta_dim_bwd[gather]");
   }
   const size_t smem = ((sizeof(float) * ((size_t)u_rows * S + (size_t)g_rows * rnd) + 15) & ~(size_t)15) + 16 * (size_t)(u_rows + g_rows);
-  TA_REQUIRE(smem <= 200 * 1024, "ta_dim_bwd: image size S=%d needs %zu B of shared memory per CTA", S, smem);
+  TA_REQUIRE(smem <= 200 * 1024, "ta_dim_bwd: image size S=%d needs %zu B of shared memory per CTA, more than the 204800 B limit", S, smem);
   auto k = tma ? dim_bwd_direct_kernel<true, false> : dim_bwd_direct_kernel<false, false>;
   static SmemOptIn optin[2] = {};
   const int rc = ensure_dyn_smem("ta_dim_bwd", k, smem, optin[tma ? 0 : 1]);
